@@ -23,6 +23,9 @@ configurations nested under "workloads" (configs[2] bpe32k_en, configs[3] bytefa
 sample_nbest64_en, and Decode(ids)) and, for N > 1, the strong-scaling run of the same 1M-sentence corpus under
 "strong_scaling".  `--workload NAME` measures one workload alone; `--scaling strong` makes the strong-scaling
 run the top-level line.  `--impl reference` times the unmodified reference on the host cores instead.
+`--dump-outputs DIR` writes what the timed path of each measured workload returned in its last timed step (rank 0's
+shard; a fixed, seeded sample of its sentences) as DIR/<workload>_<name>.npy, so that two builds can be compared
+output for output on identical inputs.
 """
 import argparse
 import ctypes
@@ -54,6 +57,11 @@ HEADLINE = "unigram32k_en"
 NESTED = ["bpe32k_en", "bytefallback_mixed", "sample_nbest64_en", "decode_unigram32k_en"]
 ENCODE_WORKLOADS = ("unigram32k_en", "bpe32k_en", "bytefallback_mixed")
 CORPUS_SEED = 20260922
+# --dump-outputs: sentences kept per workload (a fixed, seeded sample; a 1M-sentence step returns ~120 MB of ids)
+DUMP_SENTENCES = 16384
+DUMP_SEED = 20261017
+DUMP_LIMIT = 64 << 20
+_dumped = [0]
 DTYPE = "u8 text / int32 ids / f32+f64 scores"
 
 
@@ -79,6 +87,25 @@ def ids_md5(ids, ido):
     h.update(np.ascontiguousarray(ids, dtype=np.int32).tobytes())
     h.update(np.ascontiguousarray(ido, dtype=np.uint64).tobytes())
     return h.hexdigest()
+
+
+def dump_lists(args, workload, name, values, offsets):
+    """--dump-outputs: the lists values[offsets[i]:offsets[i+1]] of a fixed, seeded sample of the sentences, written as
+    <workload>_<name>.npy (float32: ids and bytes are exact in it), their lengths as <workload>_<name>_lengths.npy and
+    the sampled sentence indices as <workload>_sentences.npy (float64)."""
+    offsets = np.asarray(offsets, dtype=np.int64)
+    n = len(offsets) - 1
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_SENTENCES), replace=False))
+    lo, hi = offsets[pick], offsets[pick + 1]
+    out = {f"{workload}_sentences": pick.astype(np.float64),
+           f"{workload}_{name}_lengths": (hi - lo).astype(np.float32),
+           f"{workload}_{name}": np.concatenate([np.zeros(0)] + [values[a:b] for a, b in zip(lo, hi)]).astype(np.float32)}
+    _dumped[0] += sum(v.nbytes for v in out.values())
+    if _dumped[0] > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would exceed {DUMP_LIMIT >> 20} MB")
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
 
 
 def load_peak():
@@ -294,11 +321,12 @@ def run_reference_arm(args, rank, world):
 
 # ---------------------------------------------------------------------------------------- encode workloads ----
 
-def run_encode_workload(args, workload, rank, world, local_rank, scaling, light=False):
+def run_encode_workload(args, workload, rank, world, local_rank, scaling, light=False, dump=False):
     """One encode workload (unigram / BPE / byte-fallback).  Returns the result dict on rank 0, None elsewhere.
     scaling = "weak": every rank encodes its own `--sentences` sentences; "strong": the `--sentences` corpus of rank 0
     is cut into byte-balanced contiguous ranges (sharding.shard_ranges), one per rank.
-    light = True (nested workloads): fewer repeats of the host-side variants."""
+    light = True (nested workloads): fewer repeats of the host-side variants.
+    dump = True: the ids of the last timed step go to --dump-outputs."""
     import torch
     import torch.distributed as dist
     import corpus
@@ -451,6 +479,13 @@ def run_encode_workload(args, workload, rank, world, local_rank, scaling, light=
     ev1.record()
     sync_all()
     clocks = sampler.stop()
+    if dump and args.dump_outputs and rank == 0:
+        ids_l, offs_l = [], [np.zeros(1, np.int64)]
+        for p in slots[(step_no[0] - 1) % len(slots)]:   # the output slot of the last timed step
+            po = p["ido"][: p["n"] + 1].cpu().numpy()
+            ids_l.append(p["ids"][: int(po[-1])].cpu().numpy())
+            offs_l.append(po[1:] + offs_l[-1][-1])
+        dump_lists(args, workload, "ids", np.concatenate(ids_l), np.concatenate(offs_l))
     ms = ev0.elapsed_time(ev1)
     enc_ms = statistics.mean(all_ms)
     job_ids = total_ids
@@ -654,6 +689,8 @@ def run_decode_workload(args, rank, world, local_rank):
     text_bytes = int(to[n])
     text = np.ctypeslib.as_array(ctypes.cast(text_p, ctypes.POINTER(ctypes.c_uint8)), (max(text_bytes, 1),))[:text_bytes].copy()
     to = to.copy()
+    if args.dump_outputs and rank == 0:
+        dump_lists(args, "decode_unigram32k_en", "text", text, to)
     h2d, d2h = int(eng.info().last_h2d_bytes), int(eng.info().last_d2h_bytes)
     if world > 1:
         t = torch.tensor([dt, kernel_ms, main_ms], device=torch.device("cuda", local_rank))
@@ -737,7 +774,7 @@ def run_sample_workload(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     sampler.start()
     kernel_ms, main_ms, launches = 0.0, 0.0, 0
-    steps = min(args.steps, 5)
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         ids, ido = eng.sample_encode(buf, offs, 64, 0.5)
@@ -748,6 +785,8 @@ def run_sample_workload(args, rank, world, local_rank):
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_lists(args, "sample_nbest64_en", "ids", ids, ido)
     h2d, d2h = int(eng.info().last_h2d_bytes), int(eng.info().last_d2h_bytes)
     if world > 1:
         t = torch.tensor([dt, kernel_ms, main_ms], device=torch.device("cuda", local_rank))
@@ -814,7 +853,7 @@ def run_workload(args, name, rank, world, local_rank, scaling="weak", light=Fals
         return run_sample_workload(args, rank, world, local_rank)
     if name == "decode_unigram32k_en":
         return run_decode_workload(args, rank, world, local_rank)
-    return run_encode_workload(args, name, rank, world, local_rank, scaling, light)
+    return run_encode_workload(args, name, rank, world, local_rank, scaling, light, dump=True)
 
 
 def main():
@@ -836,6 +875,7 @@ def main():
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--warm-cache", action="store_true", help="BPE: keep the engine's word cache across steps")
     ap.add_argument("--no-nested", action="store_true", help="with --workload all: the headline workload only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of each workload's last timed step to DIR")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 

@@ -1,29 +1,29 @@
 """The drop-in caller: spm_encode_b200 (C++ host layer over the C ABI) must print exactly what the
 reference's spm_encode prints for --output_format=id / piece (BASELINE.json config 1 plumbing:
-train-on-botchan model, encode a text file, compare by md5).  Needs a B200."""
-import hashlib
+train-on-botchan model, encode a text file, compare by md5 with the reference's output, kept in
+tests/golden/reference_md5.json).  Needs a B200."""
 import os
 import subprocess
 
 import pytest
 
-from conftest import ROOT, MODELS_DIR, model_bytes
-from oracle import oracle_py
+from conftest import ROOT, MODELS_DIR
+from reference_outputs import Reference
 
 pytestmark = pytest.mark.gpu
 CLI = os.path.join(ROOT, "sentencepiece_b200", "lib", "spm_encode_b200")
 REF_CLI = os.path.join(ROOT, "oracle", "_ref", "spm_encode")
 
 
-def md5(b):
-    return hashlib.md5(b).hexdigest()
+def run_reference(args):
+    return subprocess.run([REF_CLI] + args, capture_output=True, check=True).stdout
 
 
 @pytest.mark.parametrize("model,kind,fmt,extra", [("botchan8k", "en", "id", ""), ("botchan8k", "en", "piece", ""),
                                                   ("mix_bf8k", "mixed", "id", ""), ("mix_bf8k", "mixed", "piece", ""),
                                                   ("uni32k", "mixed", "piece", "bos:eos"), ("uni32k", "mixed", "piece", "unk"),
                                                   ("bpe32k", "en", "id", "reverse:eos"), ("bpe32k", "en", "piece", "")])
-def test_cli_matches_reference(model, kind, fmt, extra, corpus_gen, tmp_path):
+def test_cli_matches_reference(model, kind, fmt, extra, corpus_gen, tmp_path, request):
     assert os.path.exists(CLI), "spm_encode_b200 has not been built (__graft_entry__.build())"
     path = str(tmp_path / "in.txt")
     n = 3000
@@ -34,16 +34,7 @@ def test_cli_matches_reference(model, kind, fmt, extra, corpus_gen, tmp_path):
     if extra:
         args.append(f"--extra_options={extra}")
     ours = subprocess.run([CLI, "--batch_lines=1000"] + args, capture_output=True, check=True).stdout
-    if os.path.exists(REF_CLI):
-        ref = subprocess.run([REF_CLI] + args, capture_output=True, check=True).stdout
-        assert md5(ours) == md5(ref), f"{model} {fmt} {extra}: output differs from the reference spm_encode"
-    elif fmt == "id" and not extra:
-        om = oracle_py.OracleModel(model_bytes(model))
-        lines = [ln for ln in open(path, "rb").read().split(b"\n")][:n]
-        exp = b"".join(b" ".join(str(i).encode() for i in om.encode(s)[0]) + b"\n" for s in lines)
-        assert md5(ours) == md5(exp)
-    else:
-        pytest.skip("oracle/_ref/spm_encode not on this box")
+    Reference(request).check("stdout", (ours,), lambda: (run_reference(args),))
 
 
 @pytest.mark.parametrize("model,kind,fmt,flags", [
@@ -57,24 +48,26 @@ def test_cli_matches_reference(model, kind, fmt, extra, corpus_gen, tmp_path):
     ("bpe32k", "en", "piece", ["--vocabulary=VOCAB", "--vocabulary_threshold=2"]),
     ("botchan8k", "en", "piece", ["--generate_vocabulary"]),
 ])
-def test_cli_formats_match_reference(model, kind, fmt, flags, corpus_gen, tmp_path):
+def test_cli_formats_match_reference(model, kind, fmt, flags, corpus_gen, tmp_path, request):
     """The other formats of spm_encode (src/spm_encode_main.cc:102-157): n-best lists, seeded sampling (the draws of a
     batch are taken in line order on one generator, like the reference's single-threaded loop), vocabulary
     restriction (:83-92) and --generate_vocabulary (:102-110,166-172)."""
     assert os.path.exists(CLI), "spm_encode_b200 has not been built (__graft_entry__.build())"
-    if not os.path.exists(REF_CLI):
-        pytest.skip("oracle/_ref/spm_encode not on this box")
+    ref = Reference(request)
     path = str(tmp_path / "in.txt")
     n = 1500
     corpus_gen.write_file(path, kind, 6262, n)
     mpath = os.path.join(MODELS_DIR, model + ".model")
     if any("VOCAB" in f for f in flags):
-        # a vocabulary file in the format --generate_vocabulary writes, made by the reference itself
+        # a vocabulary file in the format --generate_vocabulary writes, the same as the reference's own
         vpath = str(tmp_path / "vocab.tsv")
-        subprocess.run([REF_CLI, f"--model={mpath}", "--generate_vocabulary", f"--input={path}", f"--output={vpath}"], check=True)
+        gen = [f"--model={mpath}", "--generate_vocabulary", f"--input={path}"]
+        vocab = subprocess.run([CLI] + gen, capture_output=True, check=True).stdout
+        ref.check("vocabulary", (vocab,), lambda: (run_reference(gen),))
+        with open(vpath, "wb") as f:
+            f.write(vocab)
         flags = [f.replace("VOCAB", vpath) for f in flags]
     args = [f"--model={mpath}", f"--output_format={fmt}", f"--input={path}"] + flags
     ours = subprocess.run([CLI, "--batch_lines=400"] + args, capture_output=True, check=True).stdout
-    ref = subprocess.run([REF_CLI] + args, capture_output=True, check=True).stdout
     assert len(ours) > 0
-    assert md5(ours) == md5(ref), f"{model} {fmt} {flags}: output differs from the reference spm_encode"
+    ref.check("stdout", (ours,), lambda: (run_reference(args),))

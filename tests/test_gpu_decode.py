@@ -1,11 +1,12 @@
 """spm_decode_ids (K7, decode_kernel.cuh) against the oracle restatement of
-SentencePieceProcessor::Decode(ids) and, when it travelled, the live reference.  Needs a B200."""
+SentencePieceProcessor::Decode(ids) and the reference's outputs (kept as digests, tests/reference_outputs.py).  Needs a B200."""
 import numpy as np
 import pytest
 
 from conftest import model_bytes
 from oracle import modelproto as mp
 from oracle import oracle_py
+from reference_outputs import Reference
 
 pytestmark = pytest.mark.gpu
 WS = "▁"
@@ -90,15 +91,14 @@ def test_decode_toy_models_and_errors():
     assert sp.DecodeIds([ids, [b(0xE3), b(0x81), 3]]) == ["ABあZΩC��い�", "��A"]
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref did not travel to this box")
-def test_decode_vs_live_reference_large(corpus_gen):
+def test_decode_vs_live_reference_large(corpus_gen, request):
     from sentencepiece_b200 import Engine
+    ref = Reference(request)
     for model, kind in (("uni32k", "en"), ("mix_bf8k", "mixed")):
         mb = model_bytes(model)
         eng = Engine(mb)
         buf, offs = corpus_gen.fill(kind, 9202, 200000)
         ids, ido = eng.encode_packed(buf, offs)
-        text, to = eng.decode_packed(ids, ido)
-        rtext, rto = oracle_py.RefModel(mb).decode_batch(ids, ido, threads=16)
-        assert np.array_equal(to, rto) and np.array_equal(text, rtext), model
+        ref.check(f"decode_{model}", eng.decode_packed(ids, ido),
+                  lambda: oracle_py.RefModel(mb).decode_batch(ids, ido, threads=16))
         eng.close()

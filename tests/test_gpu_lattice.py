@@ -1,6 +1,6 @@
 """Full-lattice operations (SURVEY 8f item 1) through the C ABI: SampleEncode with nbest_size < 0 (forward-filtering /
 backward-sampling), SampleEncodeAndScore(wor=False) and CalculateEntropy, against the oracle (pinned against the
-reference in tests/test_oracle_lattice.py) and the live reference.  Sampled ids bit-exact under a seed (one generator,
+reference in tests/test_oracle_lattice.py) and the reference's outputs (kept as digests, tests/reference_outputs.py).  Sampled ids bit-exact under a seed (one generator,
 sentence order); sample scores and entropies within float rounding (1e-5 relative: the device's exp/log differ from
 glibc's in the last place).  Needs a B200."""
 import numpy as np
@@ -8,6 +8,7 @@ import pytest
 
 from conftest import model_bytes
 from oracle import oracle_py
+from reference_outputs import Reference
 
 pytestmark = pytest.mark.gpu
 EDGE = [b"", b"   ", b"x", b"hello world", "こんにちは \U0001F600\U0001F600 ok".encode(), b"\xff\xfe broken"]
@@ -35,16 +36,14 @@ def test_sample_lattice_seeded(model, kind, alpha, corpus_gen):
     eng.close()
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref did not travel to this box")
-def test_sample_lattice_vs_live_reference(corpus_gen):
+def test_sample_lattice_vs_live_reference(corpus_gen, request):
     lines = corpus_gen.lines("en", 9202, 40000)   # spans two chunks of the engine's lattice path
     buf, offs = oracle_py.pack(lines)
     mb = model_bytes("uni32k")
     eng = _engine("uni32k")
     eng.set_random_seed(4711)
-    ids, ido = eng.sample_encode(buf, offs, -1, 0.5)
-    rids, rido = oracle_py.RefModel(mb).sample_encode_batch(buf, offs, -1, 0.5, 4711)
-    assert np.array_equal(ido, rido) and np.array_equal(ids, rids)
+    Reference(request).check("sample", eng.sample_encode(buf, offs, -1, 0.5),
+                             lambda: oracle_py.RefModel(mb).sample_encode_batch(buf, offs, -1, 0.5, 4711))
     eng.close()
 
 

@@ -6,6 +6,7 @@ import pytest
 
 from conftest import model_bytes
 from oracle import oracle_py
+from reference_outputs import Reference
 
 pytestmark = pytest.mark.gpu
 
@@ -67,16 +68,14 @@ def test_sample_encode_seeded(model, kind, nbest, alpha, corpus_gen):
     eng.close()
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref did not travel to this box")
-def test_sample_encode_vs_live_reference(corpus_gen):
+def test_sample_encode_vs_live_reference(corpus_gen, request):
     lines = corpus_gen.lines("en", 8104, 3000)
     buf, offs = oracle_py.pack(lines)
     mb = model_bytes("uni32k")
     eng = _engine("uni32k")
     eng.set_random_seed(777)
-    ids, ido = eng.sample_encode(buf, offs, 64, 0.5)
-    rids, rido = oracle_py.RefModel(mb).sample_encode_batch(buf, offs, 64, 0.5, 777)
-    assert np.array_equal(ido, rido) and np.array_equal(ids, rids)
+    Reference(request).check("sample", eng.sample_encode(buf, offs, 64, 0.5),
+                             lambda: oracle_py.RefModel(mb).sample_encode_batch(buf, offs, 64, 0.5, 777))
     eng.close()
 
 

@@ -1,5 +1,5 @@
 """Parity of the CUDA engine (through the C ABI) with the oracle, the committed golden dumps
-of the reference, and -- when oracle/_ref travelled to this box -- the live reference.
+of the reference, and the reference's outputs on larger corpora (kept as digests, tests/reference_outputs.py).
 Bit-exact ids are required everywhere (integer/index work).  Needs a B200."""
 import base64
 import json
@@ -11,6 +11,7 @@ import pytest
 from conftest import ROOT, model_bytes
 from oracle import modelproto as mp
 from oracle import oracle_py
+from reference_outputs import Reference
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(ROOT, "tests", "golden")
@@ -254,10 +255,8 @@ def test_full_size_properties(workload, corpus_gen):
         assert ids[int(ido[i]):int(ido[i + 1])].tolist() == om.encode(s)[0].tolist(), i
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref did not travel to this box")
 @pytest.mark.parametrize("model,kind", [("uni32k", "en"), ("mix_bf8k", "mixed"), ("bpe32k", "en")])
-def test_live_reference(model, kind, corpus_gen):
+def test_live_reference(model, kind, corpus_gen, request):
     buf, offs = corpus_gen.fill(kind, 4008, 50000)
-    ids, ido = engine(model).encode_packed(buf, offs)
-    rids, rido = oracle_py.RefModel(model_bytes(model)).encode_batch(buf, offs, threads=16)
-    assert_same(ids, ido, rids, rido, f"{model}/{kind} vs live reference")
+    Reference(request).check("encode", engine(model).encode_packed(buf, offs),
+                             lambda: oracle_py.RefModel(model_bytes(model)).encode_batch(buf, offs, threads=16))

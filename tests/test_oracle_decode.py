@@ -1,13 +1,14 @@
 """Oracle restatement of SentencePieceProcessor::Decode(ids) (oracle/spm_oracle.c, oracle_decode_ids):
 the reference's own known answers (sentencepiece_processor_test.cc DecodeTest :544-640,
-ByteFallbackDecodeTest :790-900, restated over ids) and, when oracle/_ref is built, the live
-reference on round trips, random id lists and normalizer-flag variants.  CPU only."""
+ByteFallbackDecodeTest :790-900, restated over ids) and the reference's outputs (kept as digests,
+tests/reference_outputs.py) on round trips, random id lists and normalizer-flag variants.  CPU only."""
 import numpy as np
 import pytest
 
 from conftest import model_bytes
 from oracle import modelproto as mp
 from oracle import oracle_py
+from reference_outputs import Reference
 
 WS = "▁"
 N, U, C, B = mp.NORMAL, mp.UNKNOWN, mp.CONTROL, mp.BYTE
@@ -71,20 +72,19 @@ def test_out_of_range_id_fails():
         _decode(om, [-1])
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref is not built here")
 @pytest.mark.parametrize("model,kind", [("uni32k", "en"), ("mix_bf8k", "mixed"), ("bpe32k", "en"), ("mix_bpe4k", "mixed")])
-def test_oracle_decode_vs_live_reference(model, kind, corpus_gen):
+def test_oracle_decode_vs_live_reference(model, kind, corpus_gen, request):
     rng = np.random.default_rng(11)
+    ref = Reference(request)
     base = model_bytes(model)
     variants = [base, mp.replace_flags(base, add_dummy_prefix=False), mp.replace_flags(base, remove_extra_whitespaces=False),
                 mp.replace_flags(base, add_dummy_prefix=False, remove_extra_whitespaces=False)]
-    for mb in variants:
-        om, rm = oracle_py.OracleModel(mb), oracle_py.RefModel(mb)
+    for v, mb in enumerate(variants):
+        om = oracle_py.OracleModel(mb)
         buf, offs = corpus_gen.fill(kind, 9101, 1500)
-        ids, ido = rm.encode_batch(buf, offs, threads=4)
-        t1, o1 = om.decode_batch(ids, ido)
-        t2, o2 = rm.decode_batch(ids, ido, threads=4)
-        assert np.array_equal(o1, o2) and np.array_equal(t1, t2)
+        ids, ido = om.encode_batch(buf, offs)
+        ref.check(f"encode{v}", (ids, ido), lambda: oracle_py.RefModel(mb).encode_batch(buf, offs, threads=4))
+        ref.check(f"roundtrip{v}", om.decode_batch(ids, ido), lambda: oracle_py.RefModel(mb).decode_batch(ids, ido, threads=4))
         vocab = len(om.proto["pieces"])
         special = np.nonzero(np.asarray(om.proto["types"]) != mp.NORMAL)[0]
         lists = []
@@ -97,6 +97,4 @@ def test_oracle_decode_vs_live_reference(model, kind, corpus_gen):
         ido2 = np.zeros(len(lists) + 1, dtype=np.uint64)
         ido2[1:] = np.cumsum([len(x) for x in lists])
         ids2 = np.concatenate(lists)
-        t1, o1 = om.decode_batch(ids2, ido2)
-        t2, o2 = rm.decode_batch(ids2, ido2, threads=4)
-        assert np.array_equal(o1, o2) and np.array_equal(t1, t2)
+        ref.check(f"random{v}", om.decode_batch(ids2, ido2), lambda: oracle_py.RefModel(mb).decode_batch(ids2, ido2, threads=4))

@@ -1,6 +1,6 @@
 """Oracle vs outputs of the reference itself: (a) the committed golden dumps produced by
-tools/make_golden.py with the unmodified reference (oracle/_ref), (b) when oracle/_ref is
-present on this box, the live reference on fresh seeded corpora and edge cases.  CPU only."""
+tools/make_golden.py with the unmodified reference (oracle/_ref), (b) the reference's outputs
+on further seeded corpora and fuzzed inputs, kept as digests (tests/reference_outputs.py).  CPU only."""
 import base64
 import json
 import os
@@ -10,6 +10,7 @@ import pytest
 
 from conftest import ROOT, model_bytes
 from oracle import oracle_py
+from reference_outputs import Reference
 
 GOLD = os.path.join(ROOT, "tests", "golden")
 SETS = [("uni32k", "en"), ("uni32k", "mixed"), ("mix_bf8k", "mixed"), ("botchan8k", "en"), ("bpe32k", "en"),
@@ -46,53 +47,51 @@ def test_golden_edge_cases(model):
         assert (int(te[-1]) if len(te) else 0) == len(nrm)
 
 
-needs_ref = pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref not built on this box")
-
-
-@needs_ref
 @pytest.mark.parametrize("model,kind", SETS)
-def test_live_reference(model, kind, corpus_gen):
+def test_live_reference(model, kind, corpus_gen, request):
     mb = model_bytes(model)
     buf, offs = corpus_gen.fill(kind, 777, 3000)
     a, ao = oracle_py.OracleModel(mb).encode_batch(buf, offs)
-    b, bo = oracle_py.RefModel(mb).encode_batch(buf, offs, threads=4)
-    assert np.array_equal(ao, bo) and np.array_equal(a, b)
+    Reference(request).check("encode", (a, ao), lambda: oracle_py.RefModel(mb).encode_batch(buf, offs, threads=4))
 
 
-@needs_ref
 @pytest.mark.parametrize("model", ["uni32k", "bpe32k"])
-def test_live_reference_set_vocabulary(model, corpus_gen):
+def test_live_reference_set_vocabulary(model, corpus_gen, request):
     """SetVocabulary flips piece types in place (Q8); UNUSED pieces are skipped by the unigram
     Viterbi and re-split by BPE (sentencepiece_processor.cc:301-340, bpe_model.cc:175-193)."""
     mb = model_bytes(model)
-    om, rm = oracle_py.OracleModel(mb), oracle_py.RefModel(mb)
+    om, ref = oracle_py.OracleModel(mb), Reference(request)
     rng = np.random.default_rng(5)
     pieces = om.proto["pieces"]
     keep = [p for p in pieces if rng.random() < 0.5]
-    rm.set_vocabulary(keep)
-    om.set_types(om.vocabulary_types(keep))
     buf, offs = corpus_gen.fill("en", 778, 1500)
-    a, ao = om.encode_batch(buf, offs)
-    b, bo = rm.encode_batch(buf, offs)
-    assert np.array_equal(ao, bo) and np.array_equal(a, b)
-    rm.reset_vocabulary()
+
+    def reference(reset):
+        rm = oracle_py.RefModel(mb)
+        rm.set_vocabulary(keep)
+        if reset:
+            rm.reset_vocabulary()
+        return rm.encode_batch(buf, offs)
+    om.set_types(om.vocabulary_types(keep))
+    ref.check("restricted", om.encode_batch(buf, offs), lambda: reference(False))
     om.set_types(om.types)
-    a, ao = om.encode_batch(buf, offs)
-    b, bo = rm.encode_batch(buf, offs)
-    assert np.array_equal(ao, bo) and np.array_equal(a, b)
+    ref.check("reset", om.encode_batch(buf, offs), lambda: reference(True))
 
 
-@needs_ref
-def test_live_reference_normalize_alignment(corpus_gen):
+def test_live_reference_normalize_alignment(corpus_gen, request):
     mb = model_bytes("mix_bf8k")
-    om, rm = oracle_py.OracleModel(mb), oracle_py.RefModel(mb)
-    for s in corpus_gen.lines("mixed", 779, 400):
-        assert om.normalize(s) == rm.normalize(s)
+    om = oracle_py.OracleModel(mb)
+    lines = corpus_gen.lines("mixed", 779, 400)
+
+    def normalize_all(m):
+        out = [m.normalize(s) for s in lines]
+        return (b"".join(n for n, _ in out), [len(n) for n, _ in out], [len(a) for _, a in out],
+                np.concatenate([np.asarray(a, np.int64) for _, a in out]))
+    Reference(request).check("normalize", normalize_all(om), lambda: normalize_all(oracle_py.RefModel(mb)))
 
 
-@pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref is not built here")
 @pytest.mark.parametrize("model", ["uni32k", "mix_bf8k", "bpe32k", "mix_bpe4k"])
-def test_fuzz_oracle_vs_live_reference(model):
+def test_fuzz_oracle_vs_live_reference(model, request):
     """Random mixes of ASCII, runs of spaces, CJK, emoji, NFKC compatibility forms, combining marks, control bytes,
     NUL, reserved piece strings and malformed UTF-8: oracle ids (and the decoded text of those ids) == reference."""
     rng = np.random.default_rng(20260922)
@@ -107,11 +106,8 @@ def test_fuzz_oracle_vs_live_reference(model):
             parts.append(bytes(rng.integers(0, 256, size=int(rng.integers(1, 12)), dtype=np.uint8)))
         sents.append(b"".join(parts))
     mb = model_bytes(model)
-    om, rm = oracle_py.OracleModel(mb), oracle_py.RefModel(mb)
+    om, ref = oracle_py.OracleModel(mb), Reference(request)
     buf, offs = oracle_py.pack(sents)
     a, ao = om.encode_batch(buf, offs)
-    b, bo = rm.encode_batch(buf, offs, threads=8)
-    assert np.array_equal(ao, bo) and np.array_equal(a, b)
-    t1, o1 = om.decode_batch(b, bo)
-    t2, o2 = rm.decode_batch(b, bo, threads=8)
-    assert np.array_equal(o1, o2) and np.array_equal(t1, t2)
+    ref.check("encode", (a, ao), lambda: oracle_py.RefModel(mb).encode_batch(buf, offs, threads=8))
+    ref.check("decode", om.decode_batch(a, ao), lambda: oracle_py.RefModel(mb).decode_batch(a, ao, threads=8))

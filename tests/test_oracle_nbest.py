@@ -1,4 +1,5 @@
-"""Pins the oracle's n-best / sampling restatement (SURVEY 8a rows a7/a8) against the live reference:
+"""Pins the oracle's n-best / sampling restatement (SURVEY 8a rows a7/a8) against the reference's outputs
+(kept as digests, tests/reference_outputs.py):
 candidate ids, float scores bit for bit (the order among ties is libstdc++'s heap order), the agenda
 shrink path (nbest 512 on long sentences) and the seeded SampleEncode draw.  CPU only."""
 import numpy as np
@@ -7,38 +8,35 @@ import pytest
 from conftest import model_bytes
 from oracle import modelproto as mp
 from oracle import oracle_py
-
-needs_ref = pytest.mark.skipif(not oracle_py.ref_available(), reason="oracle/_ref not built on this box")
-
-
-def same_nbest(a, sa, b, sb):
-    return len(a) == len(b) and all(np.array_equal(x, y) for x, y in zip(a, b)) and \
-        np.array_equal(np.asarray(sa, np.float32).view(np.uint32), np.asarray(sb, np.float32).view(np.uint32))
+from reference_outputs import Reference
 
 
-@needs_ref
+def nbest_all(m, lines, nbest_size):
+    """n-best lists of every line, flattened: (candidates per line, ids per candidate, ids, float32 scores)"""
+    out = [m.nbest_encode(s, nbest_size) for s in lines]
+    cands = [c for cs, _ in out for c in cs]
+    return ([len(cs) for cs, _ in out], [len(c) for c in cands], np.concatenate([np.zeros(0, np.int32)] + cands),
+            np.concatenate([np.zeros(0, np.float32)] + [np.asarray(sc, np.float32) for _, sc in out]))
+
+
 @pytest.mark.parametrize("model,kind", [("uni32k", "en"), ("mix_bf8k", "mixed"), ("botchan8k", "en")])
-def test_nbest_vs_reference(model, kind, corpus_gen):
+def test_nbest_vs_reference(model, kind, corpus_gen, request):
     mb = model_bytes(model)
-    om, rm = oracle_py.OracleModel(mb), oracle_py.RefModel(mb)
+    om, ref = oracle_py.OracleModel(mb), Reference(request)
     lines = corpus_gen.lines(kind, 321, 250) + [b"", b"   ", b"a", b"hello world"]
-    for s in lines:
-        assert same_nbest(*om.nbest_encode(s, 64), *rm.nbest_encode(s, 64)), s[:60]
+    ref.check("nbest64", nbest_all(om, lines, 64), lambda: nbest_all(oracle_py.RefModel(mb), lines, 64))
     for nb in (1, 2, 5, 512, 2000):  # 512 on these sentences goes through the agenda shrink (:481-505)
-        for s in lines[:6]:
-            assert same_nbest(*om.nbest_encode(s, nb), *rm.nbest_encode(s, nb)), (nb, s[:40])
+        ref.check(f"nbest{nb}", nbest_all(om, lines[:6], nb), lambda: nbest_all(oracle_py.RefModel(mb), lines[:6], nb))
 
 
-@needs_ref
 @pytest.mark.parametrize("model,kind,nbest,alpha", [("uni32k", "en", 64, 0.5), ("mix_bf8k", "mixed", 8, 0.1)])
-def test_sample_encode_vs_reference(model, kind, nbest, alpha, corpus_gen):
+def test_sample_encode_vs_reference(model, kind, nbest, alpha, corpus_gen, request):
     mb = model_bytes(model)
     lines = corpus_gen.lines(kind, 322, 400) + [b"", b"  ", b"x"]
     buf, offs = oracle_py.pack(lines)
     for seed in (7, 4242):
-        a, ao = oracle_py.OracleModel(mb).sample_encode_batch(buf, offs, nbest, alpha, seed)
-        b, bo = oracle_py.RefModel(mb).sample_encode_batch(buf, offs, nbest, alpha, seed)
-        assert np.array_equal(ao, bo) and np.array_equal(a, b), seed
+        Reference(request).check(f"seed{seed}", oracle_py.OracleModel(mb).sample_encode_batch(buf, offs, nbest, alpha, seed),
+                                 lambda: oracle_py.RefModel(mb).sample_encode_batch(buf, offs, nbest, alpha, seed))
 
 
 # src/unigram_model_test.cc:195-238 (Viterbi / NBest on a hand-made lattice): the 2-best of "ABC" with
