@@ -26,6 +26,7 @@ enum : uint32_t {
 constexpr uint32_t kValUserDefined = 0xFFFFFFFEu;  // match-buffer marker: USER_DEFINED piece
 constexpr uint32_t kValUnk = 0xFFFFFFFDu;          // match-buffer marker: UNK edge
 constexpr uint32_t kIdxUnk = 0xFFFFFFFFu;          // DP back-pointer marker: UNK piece
+constexpr uint32_t kNoUnit = 0xFFFFFFFFu;          // KModel::ws_unit: no such trie unit
 
 // Read-only model tables resident in HBM (all L2-resident after first touch:
 // ~1 MB per model).  Pointers are device pointers.
@@ -61,6 +62,9 @@ struct KModel {
   // [trie_units] whole-word shortcut (lane_kernel.cuh): a word that is exactly the piece at this unit and ends at a normalized
   // byte position <= word_safe[unit] is certain to be encoded as that piece alone (0 = never); see engine.cu
   const uint16_t *word_safe;
+  // unigram lane kernel: trie unit of the piece path "U+2581" and its node4 entry {link, score bits, word_safe} when a
+  // walk from a U+2581 may start on that node (the nodes of E2 and E2 96 are no pieces); ws_unit = kNoUnit otherwise
+  uint32_t ws_unit, ws_link, ws_score, ws_safe;
   // [trie_units] BPE lane2 kernel: vocab id of the piece at this unit when a word that is exactly the piece encodes
   // to that single id (its merge sequence reproduces it), else 0xFFFFFFFF
   const uint32_t *word_fast;

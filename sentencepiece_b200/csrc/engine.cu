@@ -676,6 +676,28 @@ int spm_engine::upload_word_safe() {
     CUDA_TRY(d_node4.upload(n4));
     km.trie_node4 = d_node4.p;
   }
+  // Every walk of the unigram lane kernel from a U+2581 passes root -> E2 -> E2 96 -> U+2581.  When neither of the
+  // first two nodes is a piece (E2 and E2 96 are not UTF-8, so only a malformed vocabulary has them) the walk skips
+  // nothing by starting on the node of U+2581 with the piece "U+2581" relaxed, 3 bytes in (lane_kernel.cuh).
+  km.ws_unit = kNoUnit;
+  km.ws_link = km.ws_score = km.ws_safe = 0;
+  if (km.flags & kFlagFastWords) {
+    static const uint8_t kWs[3] = {0xE2, 0x96, 0x81};
+    uint32_t l = trie.link[0], v = kNoUnit;
+    for (int i = 0; i < 3; ++i) {
+      v = (l >> kLinkBaseShift) ^ kWs[i];
+      if (v >= trie.link.size() || (trie.link[v] & kLinkLabelMask) != kWs[i]) { v = kNoUnit; break; }
+      l = trie.link[v];
+      const uint32_t kind = (l >> kLinkKindShift) & 3u;
+      if (i < 2 && (kind == kKindNormal || kind == kKindUserDefined)) { v = kNoUnit; break; }
+    }
+    if (v != kNoUnit) {
+      km.ws_unit = v;
+      km.ws_link = trie.link[v];
+      km.ws_score = trie.val[v];
+      km.ws_safe = safe[v];
+    }
+  }
   return SPM_OK;
 }
 

@@ -507,6 +507,27 @@ __device__ __forceinline__ void lane_finish(const KModel &M, const KBatch &B, co
 // shared memory per warp: ring of R slots, each {score f32, back-pointer u32, position tag u16} x 32 lanes
 __host__ __device__ inline uint32_t lane_ring_bytes(uint32_t R) { return R * 32u * (4u + 4u + 2u); }
 
+// The reference's candidate score for a piece edge (unigram_model.cc:960-993) and whether it beats the value stored at
+// the target: `sc_bits` = the piece's score (NORMAL) or unused (USER_DEFINED: plen * max_score - 0.1).  Exact float
+// formulation of the mixed double comparison (Q1) when base_regular: with |score|, |base| in {0} U [2^-10, 2^18) the
+// double sum a + b is exact, so (float)cand == fl(a + b) and cand > cur <=> ns > cur || (ns == cur && err > 0), err
+// being the exact rounding error of the float add (Knuth two-sum).
+__device__ __forceinline__ bool lane_candidate(uint32_t kind, uint32_t sc_bits, uint32_t plen, float base, bool base_regular,
+                                               float curs, bool unset, float max_score, float *ns) {
+  if (kind == kKindNormal && base_regular) {
+    const float a = __uint_as_float(sc_bits);
+    *ns = __fadd_rn(a, base);
+    const float bb = __fsub_rn(*ns, a);
+    const float err = __fadd_rn(__fsub_rn(a, __fsub_rn(*ns, bb)), __fsub_rn(base, bb));
+    return unset || *ns > curs || (*ns == curs && err > 0.f);
+  }
+  const double sc = kind == kKindNormal ? static_cast<double>(__uint_as_float(sc_bits))
+                                        : static_cast<double>(__fmul_rn(static_cast<float>(plen), max_score)) - 0.1;
+  const double cand = sc + static_cast<double>(base);
+  *ns = static_cast<float>(cand);
+  return unset || cand > static_cast<double>(curs);
+}
+
 constexpr uint32_t kLogWordStep = 1u << 31;  // log entry: the previous logged position is plen bytes back (whole word)
 constexpr uint32_t kWsWord = 0x8196E2u;      // U+2581 as the low three bytes of a little-endian word
 
@@ -518,6 +539,9 @@ constexpr uint32_t kWsWord = 0x8196E2u;      // U+2581 as the low three bytes of
 // the reference necessarily ends the word with P alone.  The walk from b reaches e on P's node, P has just been
 // relaxed into e exactly as the reference relaxes it (first candidate of e), and the starts inside the word are
 // skipped: 73 % of the words of the English corpus, half of all character starts.
+// U+2581 step: every walk from a U+2581 starts with root -> E2 -> E2 96 -> U+2581, and the first two are no pieces
+// (KModel::ws_unit).  The start transition onto a U+2581 therefore puts the walk on that node at once, 3 bytes in,
+// relaxing the piece "U+2581" as the walk would: 3 of the trips of every word (~60 of 272 per English sentence) go.
 __global__ void __launch_bounds__(1024, 1) encode_unigram_lane_kernel(const KModel M, const KBatch B, uint8_t *slabs,
                                                                        uint32_t cap, uint32_t R) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -603,6 +627,31 @@ __global__ void __launch_bounds__(1024, 1) encode_unigram_lane_kernel(const KMod
       return static_cast<unsigned long long>(__funnelshift_r(w2, w3, sh)) |
              (static_cast<unsigned long long>(w3 >> sh) << 32);
     };
+    // relaxes the piece at trie unit v (kind, score bits) from s into s + plen
+    auto relax = [&](uint32_t kind, uint32_t sc_bits, uint32_t v, uint32_t plen) {
+      const uint32_t pos = s + plen;
+      uint32_t sl = ss + plen * 32u;
+      if (sl >= r_wrap) sl -= r_wrap;
+      float ns;
+      if (lane_candidate(kind, sc_bits, plen, base, base_regular, c.rs[sl], rp[sl] != pos, M.max_score, &ns)) {
+        c.rs[sl] = ns;
+        c.rb[sl] = (plen << 24) | v;
+        rp[sl] = static_cast<uint16_t>(pos);
+      }
+    };
+    // s is a U+2581 (s + 3 <= n, mblen == 3) and nothing has been walked from it: start on the node of U+2581
+    auto ws_step = [&]() {
+      k = s + 3u;
+      l = M.ws_link;
+      lsafe = M.ws_safe;
+      cur >>= 24;
+      const uint32_t kind = (M.ws_link >> kLinkKindShift) & 3u;
+      if (kind == kKindNormal || kind == kKindUserDefined) {
+        relax(kind, M.ws_score, M.ws_unit, 3u);
+        has_single = true;
+      }
+    };
+    const bool ws_on = M.ws_unit != kNoUnit;
     if (!done) {
       for (uint32_t r = 0; r < R; ++r) rp[r * 32] = 0xFFFFu;  // no slot belongs to a position of this sentence
       c.rs[0] = 0.f;
@@ -610,6 +659,7 @@ __global__ void __launch_bounds__(1024, 1) encode_unigram_lane_kernel(const KMod
       mblen = one_char_len(w0 & 0xFFu);
       if (mblen > n) mblen = n;
       cur = window_low();
+      if (ws_on && n >= 3u && (w0 & 0xFFFFFFu) == kWsWord) ws_step();
     }
     // optional counters (engine: SPM_B200_KSTATS; device-resident path only): [8] warp trips, [9] lane trips,
     // [10] starts retired, [11] whole words, [12] groups, [13] normalized bytes
@@ -638,35 +688,7 @@ __global__ void __launch_bounds__(1024, 1) encode_unigram_lane_kernel(const KMod
             const uint32_t kind = (nd.x >> kLinkKindShift) & 3u;
             if (kind == kKindNormal || kind == kKindUserDefined) {
               const uint32_t plen = k - s;
-              uint32_t sl = ss + plen * 32u;
-              if (sl >= r_wrap) sl -= r_wrap;
-              const float curs = c.rs[sl];
-              const bool unset = rp[sl] != k;
-              float ns;
-              bool better;
-              if (kind == kKindNormal && base_regular) {
-                // Exact float formulation of the reference's double comparison (Q1).  With
-                // |score|, |base| in {0} U [2^-10, 2^18) the double sum a + b is exact, so
-                // (float)cand == fl(a + b) and cand > cur <=> ns > cur || (ns == cur && err > 0),
-                // err being the exact rounding error of the float add (Knuth two-sum).
-                const float a = __uint_as_float(nd.z);
-                ns = __fadd_rn(a, base);
-                const float bb = __fsub_rn(ns, a);
-                const float err = __fadd_rn(__fsub_rn(a, __fsub_rn(ns, bb)), __fsub_rn(base, bb));
-                better = unset || ns > curs || (ns == curs && err > 0.f);
-              } else {
-                const double sc = kind == kKindNormal
-                                      ? static_cast<double>(__uint_as_float(nd.z))
-                                      : static_cast<double>(__fmul_rn(static_cast<float>(plen), M.max_score)) - 0.1;
-                const double cand = sc + static_cast<double>(base);
-                better = unset || cand > static_cast<double>(curs);
-                ns = static_cast<float>(cand);
-              }
-              if (better) {
-                c.rs[sl] = ns;
-                c.rb[sl] = (plen << 24) | v;
-                rp[sl] = static_cast<uint16_t>(k);
-              }
+              relax(kind, nd.z, v, plen);
               has_single |= plen == mblen;
             }
             // early termination: if the node has no child on the next byte the failing
@@ -755,6 +777,7 @@ __global__ void __launch_bounds__(1024, 1) encode_unigram_lane_kernel(const KMod
             k = s;
             l = root;
             has_single = false;
+            if (ws_on && wstart && s + 3u <= n) ws_step();
           }
         }
       }
